@@ -2,6 +2,7 @@
 """bench.py -- interpolated frames/sec of the RIFE hot path (BASELINE.json metric) on N B200s of one node.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 1080p|4k] [--impl ours|reference] [--scaling weak|strong]
+                  [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of synthetic frame pairs (rife-v4.6, t = 0.5): 128 pairs of 1080p, 32 of 4K.
 One invocation measures BOTH resolutions of the metric: the headline keys are BASELINE configs[1] (1920x1080), and
@@ -21,6 +22,10 @@ One invocation measures BOTH resolutions of the metric: the headline keys are BA
             launch / time; peak = measured cuBLAS bf16 TF/s.  `stages` is the per-stage breakdown of one lock-step batch.
   cpu_baseline  the reference's own CPU path (oracle/_ref: its rife.cpp CPU functions + vendored ncnn) on the host cores,
             bounded sample, rank 0 only.
+--dump-outputs DIR writes, per measured resolution, what the timed path returned in its last step: DIR/<workload>_frames_sample.npy,
+            float32, the values of a fixed sample (seed 0, DUMP_SAMPLE positions drawn with replacement, in ascending order) of
+            the step's interpolated frames, all pairs of rank 0 stacked as [pair, y, x, rgb] and flattened.  The frames are seeded
+            (synth.stream), so two builds run with the same arguments can be compared value for value.
 --impl reference times that CPU path alone on the same workload (the driver computes the ratio).
 Multi-GPU: one process per GPU (torchrun); frame pairs are independent, so ranks share nothing after rank 0 broadcasts the
 packed model over NCCL.  --scaling weak (default): fixed pairs per GPU.  --scaling strong: ONE fixed stream (256 pairs of
@@ -48,6 +53,7 @@ DISTINCT_FRAMES = 129  # consecutive frames of the synthetic stream: the default
 # a NEW frame -- pair i is (frame i, frame i + 1), so the host-buffer leg uploads pairs + 1 distinct frames per step, what a real
 # stream needs (with 9 cycling frames, as until round 2, the library's per-call frame table reduced the upload to 9 frames)
 MODEL = "rife-v4.6"
+DUMP_SAMPLE = 4 << 20  # values per resolution written by --dump-outputs: 16 MiB of float32 each, 32 MiB for both
 
 
 def measured_peaks():
@@ -229,6 +235,17 @@ def host_link_gbs():
     return out
 
 
+def dump_outputs(out_dir, workload, out_dev):
+    """The fixed sample of the frames in `out_dev` (device tensors, one per pair) described in the module docstring."""
+    import numpy as np
+    import torch
+    flat = torch.stack(out_dev).view(-1)
+    idx = np.sort(np.random.default_rng(0).integers(0, flat.numel(), min(DUMP_SAMPLE, flat.numel())))
+    vals = flat[torch.from_numpy(idx).to(flat.device)].to(torch.float32).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "%s_frames_sample.npy" % workload), vals)
+
+
 def measure(ctx, workload, args, headline):
     """All GPU-side measurements of one resolution.  Returns a dict (rank-local; times are already max-reduced over ranks)."""
     import torch
@@ -294,6 +311,8 @@ def measure(ctx, workload, args, headline):
             ev[k][1].record(stream)
         barrier()
         res["gpu_launches"] = int(pkg.launch_count() - launches0)
+    if args.dump_outputs and rank == 0 and pairs:
+        dump_outputs(args.dump_outputs, workload, out_dev)
     ms_total = reduce_max(sum(a.elapsed_time(b) for a, b in ev))
     res["ms_per_step"] = ms_total / args.steps
     res["value"] = total_pairs * args.steps / (ms_total / 1000.0)
@@ -484,6 +503,7 @@ def main():
     ap.add_argument("--timestep", type=float, default=0.5)
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU leg (and with it the parity block): profiling runs only")
     ap.add_argument("--no-process-leg", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed, seeded sample of the last timed step's frames to DIR as float32 .npy (module docstring)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

@@ -1,11 +1,16 @@
 #!/usr/bin/env python3
 """Regenerates tests/golden/golden.npz from oracle/_ref (the reference's own CPU functions + vendored ncnn, built by
-oracle/build_ref.py from /root/reference; avx2 build, the ISA every x86 CI host has).  Run here, in the container
-that holds /root/reference; the GPU box only reads the committed file.  Inputs are synth.pair(w, h, dx, dy, seed)."""
+oracle/build_ref.py from the reference's source tree; avx2 build, the ISA every x86 CI host has), where that build and the
+reference's model files are present.  Inputs are synth.pair(w, h, dx, dy, seed).
+
+--synthetic regenerates tests/golden/golden_synth.npz instead: the rife-v4.6 cases on the seeded synthetic weights of
+tests/make_synth_model.py (the model a checkout without the reference's files runs on), computed by the C++ restatement
+(oracle/build/oracle_rife), with the sha256 of the flownet.bin they were made with."""
 import hashlib
 import json
 import os
 import sys
+import tempfile
 
 import numpy as np
 
@@ -31,20 +36,31 @@ CASES = [
 ]
 
 
-def main():
+def main(synthetic=False):
     os.environ["RIFE_ORACLE_ISA"] = "avx2"
     arrays, manifest = {}, {}
+    td = tempfile.TemporaryDirectory()
+    synth_model = None
+    if synthetic:
+        import make_synth_model
+        synth_model = make_synth_model.write_model(os.path.join(td.name, "rife-v4.6"), seed=0)
     for name, model, w, h, kw, skw in CASES:
+        if synthetic and model != "rife-v4.6":
+            continue
         a, b = parity.synth.pair(w, h, **skw)
-        out, info = parity.run_oracle(model, a, b, which="ref", **kw)
+        out, info = parity.run_oracle(model, a, b, which="port" if synthetic else "ref", modeldir=synth_model, **kw)
         arrays[name] = out
         manifest[name] = {"model": model, "w": w, "h": h, "oracle_kwargs": kw, "synth_kwargs": skw,
                           "in_sha256": hashlib.sha256(a.tobytes() + b.tobytes()).hexdigest(),
                           "out_sha256": hashlib.sha256(out.tobytes()).hexdigest()}
+        if synthetic:
+            manifest[name]["model_sha256"] = parity._sha256(os.path.join(synth_model, "flownet.bin"))
         print(name, out.mean())
-    np.savez_compressed(os.path.join(HERE, "golden.npz"), **arrays)
-    json.dump(manifest, open(os.path.join(HERE, "golden.json"), "w"), indent=1, sort_keys=True)
+    base = os.path.join(HERE, "golden_synth" if synthetic else "golden")
+    np.savez_compressed(base + ".npz", **arrays)
+    json.dump(manifest, open(base + ".json", "w"), indent=1, sort_keys=True)
+    td.cleanup()
 
 
 if __name__ == "__main__":
-    main()
+    main(synthetic="--synthetic" in sys.argv[1:])

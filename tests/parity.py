@@ -1,6 +1,7 @@
 """Shared helpers for the parity tests, smoke() and bench.py's cpu_baseline leg: locate models, run the oracle
 (oracle/_ref = the reference's own CPU path when its prebuilt binary is present, else the C++ restatement in
 oracle/), run the CUDA path through the C ABI, and compare u8 frames.  TEST INFRASTRUCTURE."""
+import hashlib
 import json
 import os
 import subprocess
@@ -25,11 +26,49 @@ def model_dir(name):
     d = os.path.join(ROOT, "tests", "models", name)  # synthetic-weight models (tests/make_synth_model.py)
     if os.path.isdir(d):
         return d
-    if name == "rife-v4.6":
-        # the reference's model files did not travel: same architecture, seeded random weights (git-ignored, regenerated on demand)
-        import make_synth_model
-        return make_synth_model.write_model(d, seed=0)
+    import make_synth_model
+    if name in make_synth_model.SEEDS:
+        # the reference's model files did not travel: seeded random weights in the same file format and interface
+        # (tests/make_synth_model.py), written once per process to a temporary directory (the tree may be read-only)
+        if name not in _SYNTH:
+            if "root" not in _SYNTH:
+                import atexit
+                import shutil
+                _SYNTH["root"] = tempfile.mkdtemp(prefix="rife-b200-synth-")
+                atexit.register(shutil.rmtree, _SYNTH["root"], True)
+            _SYNTH[name] = make_synth_model.write_model(os.path.join(_SYNTH["root"], name), make_synth_model.SEEDS[name], name)
+        return _SYNTH[name]
     return None
+
+
+_SYNTH = {}
+GOLD_DIR = os.path.join(ROOT, "tests", "golden")
+
+
+def _sha256(path):
+    h = hashlib.sha256()
+    with open(path, "rb") as f:
+        for chunk in iter(lambda: f.read(1 << 20), b""):
+            h.update(chunk)
+    return h.hexdigest()
+
+
+def golden_frame(name):
+    """The committed golden frame of case `name` (tests/golden/golden.json) for the model files model_dir() finds, or None
+    when there is none for them.  golden.npz holds the reference's CPU path on the reference's model files;
+    golden_synth.npz holds the C++ restatement (oracle/) on the seeded synthetic rife-v4.6 weights of
+    tests/make_synth_model.py, which stand in where the reference's files are absent.  The synthetic set is chosen only
+    when the flownet.bin in use is byte for byte the one it was made with."""
+    m = json.load(open(os.path.join(GOLD_DIR, "golden.json")))[name]
+    md = model_dir(m["model"])
+    if md is None:
+        return None
+    synth = json.load(open(os.path.join(GOLD_DIR, "golden_synth.json"))).get(name)
+    if synth is not None and _sha256(os.path.join(md, "flownet.bin")) == synth["model_sha256"]:
+        return np.load(os.path.join(GOLD_DIR, "golden_synth.npz"))[name]
+    if md == _SYNTH.get(m["model"]):  # a generated stand-in without committed frames of its own
+        return None
+    return np.load(os.path.join(GOLD_DIR, "golden.npz"))[name]
 
 
 def _cpu_flags():
