@@ -120,7 +120,7 @@ int rife_b200_bench_conv_batched(int gpuid, void* cuda_stream, int cin, int cout
 
 /* Diagnostics: clock64 timeline (64 slots per CTA) of one tcgen05 conv launch; see csrc/tc_conv.cu for the slot map.
  * `split`: bit 0 = split hi+lo operands, bits 8-15 = images per launch (0 = 1), bits 16-23 = tiles each CTA skips
- * before recording (steady state instead of pipeline fill). */
+ * before recording (steady state instead of pipeline fill); the bits above must be 0 (RIFE_B200_ERR_ARG otherwise). */
 int rife_b200_debug_conv_timeline(int gpuid, int cin, int cout, int h, int w, int split, unsigned long long* host_out,
                                   int max_ctas);
 
@@ -154,7 +154,8 @@ int rife_b200_debug_parse_model(const char* param_path, const char* bin_path, in
 /* Diagnostics (host only, no GPU): the weight packing of the tcgen05 kernel, fp16 bit patterns.
  * mode 0: conv3x3 w[cout][cin][3][3]; mode 1: deconv4x4 s2 w[cout][cin][4][4] with `ocs` column slots per output parity.
  * out_elems must be (cin/16)*9*2*N*8.  paired: 0 = [kc][tap][half][N][8]; 1 = [kc][dx][half][3N: dy2|dy0|dy1][8]
- * (the layout of the paired MMA issue, 2N <= 256); -1 = whatever this process uses (environment RIFE_B200_PAIR). */
+ * (the layout of the paired MMA issue; with 2N > 256 the layout of 0); -1 = what the kernel uses for this N (1 when
+ * 2N <= 256, else 0).  Any other value returns RIFE_B200_ERR_ARG. */
 int rife_b200_debug_pack_weights(int mode, int cout, int cin, int N, int ocs, int paired, const float* w,
                                  unsigned short* out, size_t out_elems);
 

@@ -192,11 +192,11 @@ def bench_conv(cuda_stream_ptr, cin, cout, h, w, split, iters, gpuid=0, batch=1)
         raise RifeError("bench_conv failed: %d" % rc)
 
 
-def debug_conv_timeline(cin, cout, h, w, split=True, max_ctas=148, gpuid=0, batch=1, skip_tiles=0, flags=0):
+def debug_conv_timeline(cin, cout, h, w, split=True, max_ctas=148, gpuid=0, batch=1, skip_tiles=0):
     buf = np.zeros((max_ctas, 64), np.uint64)
     L = lib()
     L.rife_b200_debug_conv_timeline.argtypes = [ctypes.c_int] * 6 + [ctypes.c_void_p, ctypes.c_int]
-    rc = L.rife_b200_debug_conv_timeline(gpuid, cin, cout, h, w, int(bool(split)) | (int(batch) << 8) | (int(skip_tiles) << 16) | (int(flags) << 24), buf.ctypes.data, max_ctas)
+    rc = L.rife_b200_debug_conv_timeline(gpuid, cin, cout, h, w, int(bool(split)) | (int(batch) << 8) | (int(skip_tiles) << 16), buf.ctypes.data, max_ctas)
     if rc != 0:
         raise RifeError("debug_conv_timeline failed: %d" % rc)
     return buf

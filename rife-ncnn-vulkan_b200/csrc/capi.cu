@@ -375,7 +375,7 @@ extern "C" int rife_b200_debug_parse_model(const char* param_path, const char* b
 extern "C" int rife_b200_debug_pack_weights(int mode, int cout, int cin, int N, int ocs, int paired, const float* w, unsigned short* out, size_t out_elems) {
     GUARD_BEGIN
     using namespace rife;
-    if (!w || !out || cin % 16 || N % 16 || cout <= 0 || cout > N) return RIFE_B200_ERR_ARG;
+    if (!w || !out || cin % 16 || N % 16 || cout <= 0 || cout > N || paired < -1 || paired > 1) return RIFE_B200_ERR_ARG;
     std::vector<uint16_t> pk;
     if (mode == 0) pack_conv3x3_weights(w, cout, cin, N, pk, paired);
     else if (mode == 1) { if (4 * ocs > N || cout > ocs) return RIFE_B200_ERR_ARG; pack_deconv4x4_weights(w, cout, cin, ocs, N, pk, paired); }
@@ -398,27 +398,25 @@ extern "C" int rife_b200_set_stream(rife_b200_t* h, void* cuda_stream) {
 }
 
 static unsigned long long* g_dbg_dev = nullptr;
-static int g_dbg_skip = 0, g_dbg_flags = 0;
+static int g_dbg_skip = 0;
 
 // diagnostics: per-CTA clock64 timeline of one tcgen05 conv launch (64 slots per CTA, see tc_conv.cu)
 extern "C" int rife_b200_debug_conv_timeline(int gpuid, int cin, int cout, int h, int w, int split, unsigned long long* host_out, int max_ctas) {
     GUARD_BEGIN
-    if (!host_out || max_ctas <= 0) return RIFE_B200_ERR_ARG;
+    if (!host_out || max_ctas <= 0 || (split >> 24) != 0) return RIFE_B200_ERR_ARG;
     if (cudaSetDevice(gpuid) != cudaSuccess) return RIFE_B200_ERR_DEVICE;
     size_t bytes = (size_t)max_ctas * 64 * 8;
     cudaMalloc(&g_dbg_dev, bytes);
     cudaMemset(g_dbg_dev, 0, bytes);
-    // split: bit 0 = split operands, bits 8-15 = images per launch (0 -> 1), bits 16-23 = tiles to skip before recording
+    // split: bit 0 = split operands, bits 8-15 = images per launch (0 -> 1), bits 16-23 = tiles to skip before recording, bits 24-31 = 0
     const int batch = ((split >> 8) & 0xff) ? ((split >> 8) & 0xff) : 1;
     g_dbg_skip = (split >> 16) & 0xff;
-    g_dbg_flags = (split >> 24) & 0x7f;  // epilogue knock-outs, see TcConvArgs::dbg_flags
     int r = rife_b200_bench_conv_batched(gpuid, nullptr, cin, cout, h, w, split & 1, batch, 3);  // warm (dbg active on every launch; last one kept)
     cudaDeviceSynchronize();
     cudaMemcpy(host_out, g_dbg_dev, bytes, cudaMemcpyDeviceToHost);
     cudaFree(g_dbg_dev);
     g_dbg_dev = nullptr;
     g_dbg_skip = 0;
-    g_dbg_flags = 0;
     return r;
     GUARD_END
 }
@@ -464,9 +462,6 @@ extern "C" int rife_b200_bench_conv_batched(int gpuid, void* cuda_stream, int ci
     a.H = h; a.W = w; a.Cin = cin; a.Cout = cout; a.N = cout; a.split_in = split; a.split_out = split; a.epi = TC_EPI_C8; a.act_mode = 1;
     a.dbg = g_dbg_dev;
     a.dbg_skip = g_dbg_skip;
-    a.dbg_flags = g_dbg_flags;
-    // knock-out timing without the in-kernel timeline (tools/knockout.py): RIFE_B200_DBG_FLAGS is read on every call
-    if (!g_dbg_dev) if (const char* e = getenv("RIFE_B200_DBG_FLAGS")) a.dbg_flags = atoi(e);
     if (batch > 1) {
         // reinterpret the tall synthetic tensor as `batch` images: per image [planes][C/8][h/batch][w][8]; the values are
         // arbitrary, only the addressing pattern matters for timing

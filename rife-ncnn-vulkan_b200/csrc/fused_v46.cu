@@ -251,9 +251,6 @@ int V46Runner::conv(int slot, const __half* in, __half* out, const __half* res, 
     a.s2 = W.tc_s2;
     a.num_sms = wr_->num_sms;
     a.batch = batch;
-    // consecutive convolutions of a block walk their tiles in opposite directions: each starts with what its producer wrote last,
-    // i.e. with the part of its input that is still in L2 (the head kernel before conv0 runs in natural order, so conv0 is reversed)
-    a.rev = snake_ ? ((slot % 11 + 1) & 1) : 0;
     a.in_bstride = (size_t)(W.tc_s2 ? 4 : 1) * W.cinp * oh * ow * 2;  // room for hi + lo planes of one image (also when only hi is used)
     if (L.type == "Convolution") {
         a.out_bstride = a.res_bstride = (size_t)L.geti(0, 0) * oh * ow * 2;

@@ -4,8 +4,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <stdlib.h>
-
 #include <string>
 #include <vector>
 
@@ -70,8 +68,7 @@ private:
     uchar4* rgbx_ = nullptr;  // the distinct frames of a batch, padded RGBX
     float *F_ = nullptr, *M_ = nullptr, *d_[4] = {};
     __half *x_[4] = {}, *y0_[4] = {}, *a_[4] = {}, *b_[4] = {}, *c_[4] = {};
-    bool res_split_ = false;
-    int snake_ = getenv("RIFE_B200_SNAKE") ? atoi(getenv("RIFE_B200_SNAKE")) : 0;  // alternate the tile direction of consecutive convolutions  // the residual handed to conv() carries a lo plane
+    bool res_split_ = false;  // the residual handed to conv() carries a lo plane
 };
 
 }  // namespace rife

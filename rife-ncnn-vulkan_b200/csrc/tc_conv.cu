@@ -18,7 +18,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
-#include <stdlib.h>
 
 #include <mutex>
 #include <type_traits>
@@ -177,14 +176,7 @@ __device__ __forceinline__ uint32_t pack2(__half a, __half b) { return (uint32_t
 // input (4 parity sub-images [py][px] of H/2 x W/2, each a run of K chunks): input row 2y+dy-1 is row y-1 of the odd
 // sub-image for dy = 0, row y of the even one for dy = 1 and row y of the odd one for dy = 2 (columns alike), so a
 // chunk of parity (py,px) contributes (py?2:1)*(px?2:1) taps, each again a plain shifted view of the same slab.
-// WIDE = 1 (stride-1 convs with 3N <= 256): an accumulator is 128 consecutive pixels of ONE image row instead of 2 rows x 64,
-// the tile is MT rows x 126 columns.  Halo row r is then the dy operand of accumulator r - dy for all three dy, and those
-// accumulators are adjacent in TMEM: ONE MMA of up to 3N columns against [W_dy2 | W_dy1 | W_dy0] updates all of them, so a
-// kernel column costs MT + 2 MMAs instead of 3 MT (2 MT + 1 with the paired issue) and every activation row is fetched from
-// shared memory once instead of three (two) times -- the mainloop of the N <= 64 layers is bound by exactly that fetch
-// (profiles/README.md).  The wrap-around of a shifted 128-pixel view into the next row only reaches output columns 126, 127,
-// which are not stored.
-template <int N, int MT, int STAGES, int TAPS, int WIDE>
+template <int N, int MT, int STAGES, int TAPS>
 __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_constant__ CUtensorMap tmA, TcConvArgs a) {
     // TAPS = 5: a 5x5 stride-1 pad-2 convolution, one KERNEL ROW per pipeline stage.  The K loop runs over (16-channel chunk,
     // dy): a stage carries the 2*MT image rows that tap row dy reads (no halo rows: the next dy re-loads the rows shifted by
@@ -192,12 +184,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
     // The tile keeps 60 valid columns (halo 2 left and right).  All 25 taps of a chunk in one stage would need up to 150 KB of
     // weights per stage (N = 192); a row is 31 KB.
     constexpr int HALO = TAPS == 5 ? 2 : 1;
-    constexpr int TWP = WIDE ? 128 : 64;          // tile width incl. the halo columns left and right
+    constexpr int TWP = 64;                       // tile width incl. the halo columns left and right
     constexpr int TVALID = TWP - 2 * HALO;
-    constexpr int RPA = WIDE ? 1 : 2;             // image rows per accumulator
-    constexpr int ROWS = TAPS == 5 ? 2 * MT : RPA * MT + 2;  // input rows per stage (3x3: halo rows included)
+    constexpr int ROWS = TAPS == 5 ? 2 * MT : 2 * MT + 2;  // input rows per stage (3x3: halo rows included)
     constexpr int A_PLANE = 2 * ROWS * TWP * 16;  // bytes of one plane slab: 2 eight-channel halves
-    static_assert(!WIDE || (TAPS == 9 && 3 * N <= 256), "wide tiles: stride-1 convs whose three row taps fit one MMA");
     constexpr int W_BYTES = TAPS * 2 * N * 16;
     constexpr int ACC_COLS = MT * N;              // TMEM columns per accumulator set
     static_assert(2 * ACC_COLS <= 512, "TMEM overflow");
@@ -219,21 +209,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
     uint64_t* acc_full = empty + 8;
     uint64_t* acc_empty = acc_full + 2;
     uint64_t* wbar = acc_empty + 2;
-    uint64_t* scratch_bar = wbar + 1;  // diagnostics only (dbg_flags 64)
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(scratch_bar + 1);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wbar + 1);
     float* slope_s = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(full) + 256);  // per-channel (slope - 1), PReLU epilogue only; 16-byte aligned
     // Constant MMA operands, built once per CTA:
     //  ones  : A tile 128 x 16 with K columns 0..2 = 1      }  first MMA of every tile: D = ones * biasB = the fp32 bias
     //  biasB : B tile 16 x N, K rows 0..2 = bias as hi+lo+lo2 }  (three fp16 pieces), so no epilogue touches the bias
     //  ident : res_mode 3 (residual == this conv's own input): the residual is added by the tensor core as a tenth tap
-    //          whose B operand is an identity slice.  K-major matrix of IROWS rows with ones at rows N-16 .. N-1 (row
-    //          N-16+k has its one in K column k); the B view of K chunk kc starts (N-16-16*kc) rows in, which puts the
-    //          ones at columns n = 16*kc + k.  The centre view of the halo tile is the A operand: no global residual read.
-    constexpr int IROWS = 2 * N - 16;
+    //          whose B operand is a 16 x 16 identity; the MMA of K chunk kc targets only the 16 accumulator columns of that
+    //          chunk's channels.  The centre view of the halo tile is the A operand: no global residual read.
+    //          Only 2 x 16 x 16 B of IDENT_BYTES are used; the region stays larger on purpose (see launch_t).
+    constexpr int IDENT_BYTES = 2 * (2 * N - 16) * 16;
     __half* ones = reinterpret_cast<__half*>(smem + (size_t)NST * stage_bytes + 1024 + 256 + N * sizeof(float));
     __half* biasB = ones + 2 * 128 * 8;
     __half* ident = biasB + 2 * N * 8;
-    uint8_t* wres = smem + (((size_t)NST * stage_bytes + 1024 + 256 + N * sizeof(float) + 2 * 128 * 16 + 2 * N * 16 + 2 * IROWS * 16 + 127) & ~(size_t)127);
+    uint8_t* wres = smem + (((size_t)NST * stage_bytes + 1024 + 256 + N * sizeof(float) + 2 * 128 * 16 + 2 * N * 16 + IDENT_BYTES + 127) & ~(size_t)127);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tiles_img = a.tiles_x * a.tiles_y;
@@ -241,13 +230,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
     const int KCP = a.Cin / 16;                    // K chunks per parity sub-image (all of them for stride 1)
     const int KC = TAPS == 9 ? KCP : (TAPS == 5 ? 5 * KCP : 4 * KCP);
     const uint32_t dskip = (uint32_t)(a.dbg_skip * KC);  // diagnostics: first recorded pipeline iteration
-    const int krot = a.krot ? (int)((blockIdx.x * 5u) % (unsigned)KC) : 0;
 
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < NST; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
         for (int s = 0; s < 2; s++) { mbar_init(&acc_full[s], 1); mbar_init(&acc_empty[s], 8); }
         mbar_init(wbar, 1);
-        mbar_init(scratch_bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
     }
@@ -275,17 +262,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
         }
         *reinterpret_cast<uint4*>(biasB + (size_t)i * 8) = z;
     }
-    if (a.res_mode == 3 && ((a.pair & 2) || WIDE)) {
-        // narrow identity tap: a 16 x 16 identity [half][16 rows][8]; the MMA of K chunk kc targets only the 16 accumulator
-        // columns of that chunk's channels (N = 16 instead of N: a quarter of the B bytes, a quarter of the math)
+    if (a.res_mode == 3) {
+        // 16 x 16 identity [half][16 rows][8]
         for (int i = threadIdx.x; i < 2 * 16 * 8; i += NTHREADS) {
             const int j = i & 7, r = (i >> 3) & 15, hf = i >> 7;
             ident[i] = __float2half_rn(r == hf * 8 + j ? 1.f : 0.f);
-        }
-    } else if (a.res_mode == 3) {
-        for (int i = threadIdx.x; i < 2 * IROWS * 8; i += NTHREADS) {
-            const int j = i & 7, r = (i >> 3) % IROWS, hf = (i >> 3) / IROWS;
-            ident[i] = __float2half_rn(r - (N - 16) == hf * 8 + j ? 1.f : 0.f);
         }
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the tensor core
@@ -312,22 +293,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                 for (int kc = 0; kc < KC; kc++) bulk_load_1d(wres + (size_t)kc * W_BYTES, a.wpk + (size_t)kc * (W_BYTES / 2), W_BYTES, wbar);
             }
             for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-                // a.rev: this launch walks the tiles in reverse raster order.  Consecutive layers of a chain alternate, so a layer
-                // starts with the part of its input the previous layer wrote last -- the part still in the 126 MB L2
-                const int teff = a.rev ? ntiles - 1 - tile : tile;
-                const int bimg = teff / tiles_img, trem = teff - bimg * tiles_img;
+                const int bimg = tile / tiles_img, trem = tile - bimg * tiles_img;
                 const int tx = trem % a.tiles_x, ty = trem / a.tiles_x;
-                const int x0 = tx * TVALID, y0 = ty * (RPA * MT);
-                for (int kk = 0, q = 0; kk < KC; kk++, it++) {
-                    // a.krot (streamed weights): every CTA starts its K loop at a different chunk, so the CTAs of a wave do not all
-                    // ask L2 for the same weight lines at the same moment (accumulation order is free: the bias MMA comes first)
-                    const int kc = kk + krot < KC ? kk + krot : kk + krot - KC;
-                    if (a.dbg_flags & 16) {  // timing experiment: no loads at all (the MMAs read whatever the slabs hold)
-                        if (q == 0) mbar_wait(&empty[s], ph ^ 1);
-                        if (q == KS - 1) mbar_arrive(&full[s]);
-                        if (++q == KS) { q = 0; if (++s == NST) { s = 0; ph ^= 1; } }
-                        continue;
-                    }
+                const int x0 = tx * TVALID, y0 = ty * (2 * MT);
+                for (int kc = 0, q = 0; kc < KC; kc++, it++) {
                     if (q == 0) {
                         mbar_wait(&empty[s], ph ^ 1);
                         mbar_arrive_expect_tx(&full[s], (uint32_t)(KS * (A_PLANE * nplanes + (a.wres ? 0 : W_BYTES))));
@@ -335,7 +304,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                     uint8_t* st = smem + (size_t)s * stage_bytes + (size_t)q * sub_bytes;
                     for (int p = 0; p < nplanes; p++) {
                         if constexpr (TAPS == 5) tma_load_4d(st + p * A_PLANE, &tmA, &full[s], (x0 - 2) * 4, y0 - 2 + kc % 5, p * (2 * KCP) + 2 * (kc / 5), bimg);
-                        else tma_load_4d(st + p * A_PLANE, &tmA, &full[s], (x0 - 1) * (WIDE ? 2 : 4), y0 - 1, p * (2 * KC) + 2 * kc, bimg);  // 16 B per pixel = 4 u32 / 2 u64 elements
+                        else tma_load_4d(st + p * A_PLANE, &tmA, &full[s], (x0 - 1) * 4, y0 - 1, p * (2 * KC) + 2 * kc, bimg);  // 16 B per pixel = 4 u32 elements
                     }
                     if (!a.wres) bulk_load_1d(st + nplanes * A_PLANE, a.wpk + (size_t)kc * (W_BYTES / 2), W_BYTES, &full[s]);
                     if (dbg && it - dskip < 12u) dbg[1 + it - dskip] = clock64();
@@ -372,10 +341,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                     const uint32_t bb_lo = (smem_u32(biasB) >> 4) | B_LBO;
 #pragma unroll
                     for (int m = 0; m < MT; m++)
-                        if (!(a.dbg_flags & 2) || tcount < 2) umma_f16_elect(acc0 + m * N, o_lo, DESC_HI, bb_lo, DESC_HI, idesc, 0u);  // (flag 2: timing experiment, bias MMAs only on the first use of each buffer)
+                        umma_f16_elect(acc0 + m * N, o_lo, DESC_HI, bb_lo, DESC_HI, idesc, 0u);
                 }
-                for (int kk = 0, q = 0; kk < KC; kk++, it++) {
-                    const int kc = kk + krot < KC ? kk + krot : kk + krot - KC;  // same rotation as the producer
+                for (int kc = 0, q = 0; kc < KC; kc++, it++) {
                     if (q == 0) {
                         mbar_wait(&full[s], ph);
                         tc_fence_after();
@@ -384,29 +352,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                     const uint32_t st = smem_u32(smem + (size_t)s * stage_bytes + (size_t)q * sub_bytes);
                     const uint32_t a_base = (st >> 4) | A_LBO;
                     const uint32_t b_base = ((a.wres ? wres_addr + (uint32_t)(kc * W_BYTES) : st + nplanes * A_PLANE) >> 4) | B_LBO;
-                    constexpr int ROWSTEP16 = (RPA * TWP * 16) >> 4;  // accumulator m+1 starts RPA tile rows further
-                    if constexpr (WIDE) {
-                        constexpr uint32_t B3_LBO = ((uint32_t)(3 * N * 16) >> 4) << 16;
-                        constexpr uint32_t idesc2 = (1u << 4) | ((uint32_t)((2 * N) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-                        constexpr uint32_t idesc3 = (1u << 4) | ((uint32_t)((3 * N) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-                        const uint32_t b_addr = a.wres ? wres_addr + (uint32_t)(kc * W_BYTES) : st + nplanes * A_PLANE;
-#pragma unroll
-                        for (int dx = 0; dx < 3; dx++) {  // weight block of (kc, dx): [half][3N rows: dy2 | dy1 | dy0][8] (to_wide_layout)
-                            const uint32_t b_lo = ((b_addr + (uint32_t)(dx * (2 * 3 * N * 16))) >> 4) | B3_LBO;
-                            const uint32_t a_lo = a_base + (uint32_t)dx;
-                            if (nplanes == 2) umma_issue_wide<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, idesc2, idesc3, 1u);
-                            else umma_issue_wide<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, idesc2, idesc3, 1u);
-                        }
-                        if (a.res_mode == 3) {  // the self-residual as a narrow identity tap onto the 16 accumulator columns of this K chunk
-                            constexpr uint32_t I16_LBO = ((uint32_t)(16 * 16) >> 4) << 16;
-                            constexpr uint32_t idesc16 = (1u << 4) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-                            const uint32_t b_lo = (smem_u32(ident) >> 4) | I16_LBO;
-                            const uint32_t a_lo = a_base + (uint32_t)(((1 * TWP + 1) * 16) >> 4);
-                            const uint32_t accn = acc0 + (uint32_t)(16 * kc);
-                            if (nplanes == 2) umma_issue_tap<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(accn, a_lo, b_lo, DESC_HI, idesc16, 1u);
-                            else umma_issue_tap<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(accn, a_lo, b_lo, DESC_HI, idesc16, 1u);
-                        }
-                    } else if constexpr (TAPS == 5) {
+                    constexpr int ROWSTEP16 = (2 * TWP * 16) >> 4;  // accumulator m+1 starts 2 tile rows further
+                    if constexpr (TAPS == 5) {
 #pragma unroll
                         for (int dx = 0; dx < 5; dx++) {  // the five taps of kernel row kc % 5
                             const uint32_t b_lo = b_base + (uint32_t)(dx * (2 * N * 16) >> 4);
@@ -414,75 +361,31 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                             if (nplanes == 2) umma_issue_tap<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, 1u);
                             else umma_issue_tap<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, 1u);
                         }
+                    } else if constexpr (TAPS == 9 && tc_paired(N)) {
+                        // Paired issue: the view of halo rows 2j, 2j+1 is the dy=0 operand of accumulator j AND the dy=2 operand of
+                        // accumulator j-1, whose TMEM columns are adjacent -- one 2N-column MMA against [W_dy2 | W_dy0] replaces two
+                        // N-column ones (A is fetched from shared memory once instead of twice; 2*MT+1 MMAs per kernel column instead
+                        // of 3*MT).  Weight block of (kc, dx): [half][3N rows: dy2 | dy0 | dy1][8] (to_paired_layout).  res_mode 3
+                        // adds the identity tap onto the 16 accumulator columns of this chunk's channels.  Every MMA of the chunk is
+                        // issued from ONE asm block with literal operand offsets (tools/gen_mma_issue.py chunk_block).
+                        constexpr uint32_t B3_LBO = ((uint32_t)(3 * N * 16) >> 4) << 16;
+                        constexpr uint32_t idesc2 = (1u << 4) | ((uint32_t)((2 * N) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+                        constexpr uint32_t I16_LBO = ((uint32_t)(16 * 16) >> 4) << 16;
+                        constexpr uint32_t idesc16 = (1u << 4) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+                        const uint32_t b_addr = a.wres ? wres_addr + (uint32_t)(kc * W_BYTES) : st + nplanes * A_PLANE;
+                        const uint32_t b_lo = (b_addr >> 4) | B3_LBO;
+                        const uint32_t id_lo = (smem_u32(ident) >> 4) | I16_LBO;
+                        const uint32_t id_on = a.res_mode == 3 ? 1u : 0u;
+                        if (nplanes == 2) umma_issue_chunk_paired<N, MT, 2>(acc0, a_base, b_lo, DESC_HI, idesc, idesc2, id_on, id_lo, idesc16, acc0 + (uint32_t)(16 * kc));
+                        else umma_issue_chunk_paired<N, MT, 1>(acc0, a_base, b_lo, DESC_HI, idesc, idesc2, id_on, id_lo, idesc16, acc0 + (uint32_t)(16 * kc));
                     } else if constexpr (TAPS == 9) {
-                        bool paired = false;
-                        if constexpr (2 * N <= 256) paired = (a.pair & 1) != 0;
-                        bool chunk_block = false;
-                        if constexpr (2 * N <= 256 && (N <= 64 || N == 96 || N == 128) && (N % 16 == 0) && !(N > 64 && MT != 2) && !(N <= 64 && MT != 4)) {
-                            // the shipped path: every MMA of the chunk in ONE asm block with literal operand offsets (tools/gen_mma_issue.py
-                            // chunk_block); the per-tap blocks below remain for the diagnostic knock-outs and the unpaired layout
-                            chunk_block = paired && a.dbg_flags == 0 && a.chunk_issue && (a.res_mode != 3 || (a.pair & 2));
-                            if (chunk_block) {
-                                constexpr uint32_t B3_LBO = ((uint32_t)(3 * N * 16) >> 4) << 16;
-                                constexpr uint32_t idesc2 = (1u << 4) | ((uint32_t)((2 * N) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-                                constexpr uint32_t I16_LBO = ((uint32_t)(16 * 16) >> 4) << 16;
-                                constexpr uint32_t idesc16 = (1u << 4) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-                                const uint32_t b_addr = a.wres ? wres_addr + (uint32_t)(kc * W_BYTES) : st + nplanes * A_PLANE;
-                                const uint32_t b_lo = (b_addr >> 4) | B3_LBO;
-                                const uint32_t id_lo = (smem_u32(ident) >> 4) | I16_LBO;
-                                const uint32_t id_on = a.res_mode == 3 ? 1u : 0u;
-                                if (nplanes == 2) umma_issue_chunk_paired<N, MT, 2>(acc0, a_base, b_lo, DESC_HI, idesc, idesc2, id_on, id_lo, idesc16, acc0 + (uint32_t)(16 * kc));
-                                else umma_issue_chunk_paired<N, MT, 1>(acc0, a_base, b_lo, DESC_HI, idesc, idesc2, id_on, id_lo, idesc16, acc0 + (uint32_t)(16 * kc));
-                            }
-                        }
-                        if (chunk_block) {
-                        } else if (paired) {
-                            // Paired issue: the view of halo rows 2j, 2j+1 is the dy=0 operand of accumulator j AND the dy=2
-                            // operand of accumulator j-1, whose TMEM columns are adjacent -- one 2N-column MMA against
-                            // [W_dy2 | W_dy0] replaces two N-column ones (A is fetched from shared memory once instead of
-                            // twice; 2*MT+1 MMAs per kernel column instead of 3*MT).  Weight block of (kc, dx):
-                            // [half][3N rows: dy2 | dy0 | dy1][8] (to_paired_layout).
-                            if constexpr (2 * N <= 256) {
-                                constexpr uint32_t B3_LBO = ((uint32_t)(3 * N * 16) >> 4) << 16;
-                                constexpr uint32_t idesc2 = (1u << 4) | ((uint32_t)((2 * N) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-                                const uint32_t b_addr = a.wres ? wres_addr + (uint32_t)(kc * W_BYTES) : st + nplanes * A_PLANE;
+                        // 2N > 256 (N = 192): nine N-column taps over [tap][half][N][8] weights; the launcher never selects the
+                        // identity tap for these layers
 #pragma unroll
-                                for (int dx = 0; dx < 3; dx++) {
-                                    if ((a.dbg_flags & 4) && dx > 0) continue;  // timing experiment: a third of the taps (results wrong)
-                                    const uint32_t b_lo = ((b_addr + (uint32_t)(dx * (2 * 3 * N * 16))) >> 4) | B3_LBO;
-                                    const uint32_t a_lo = a_base + (uint32_t)dx;
-                                    if (nplanes == 2) {
-                                        umma_issue_pair<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, idesc2, 1u);
-                                        umma_issue_tap<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo + (uint32_t)TWP, b_lo + (uint32_t)(2 * N), DESC_HI, idesc, 1u);
-                                    } else {
-                                        umma_issue_pair<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, idesc2, 1u);
-                                        umma_issue_tap<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo + (uint32_t)TWP, b_lo + (uint32_t)(2 * N), DESC_HI, idesc, 1u);
-                                    }
-                                }
-                            }
-                        } else {
-#pragma unroll
-                            for (int tap = 0; tap < 9; tap++) {
-                                const int dy = tap / 3, dx = tap - dy * 3;
-                                const uint32_t b_lo = b_base + (uint32_t)(tap * (2 * N * 16) >> 4);
-                                const uint32_t a_lo = a_base + (uint32_t)(((dy * TWP + dx) * 16) >> 4);
-                                if (nplanes == 2) umma_issue_tap<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, 1u);
-                                else umma_issue_tap<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, 1u);
-                            }
-                        }
-                        if (chunk_block) {
-                        } else if (a.res_mode == 3 && (a.pair & 2) && !(a.dbg_flags & 1)) {  // (flag 1: timing experiment without the identity tap)
-                            constexpr uint32_t I16_LBO = ((uint32_t)(16 * 16) >> 4) << 16;
-                            constexpr uint32_t idesc16 = (1u << 4) | ((uint32_t)(16 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-                            const uint32_t b_lo = (smem_u32(ident) >> 4) | I16_LBO;
-                            const uint32_t a_lo = a_base + (uint32_t)(((1 * TWP + 1) * 16) >> 4);
-                            const uint32_t accn = acc0 + (uint32_t)(16 * kc);
-                            if (nplanes == 2) umma_issue_tap<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(accn, a_lo, b_lo, DESC_HI, idesc16, 1u);
-                            else umma_issue_tap<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(accn, a_lo, b_lo, DESC_HI, idesc16, 1u);
-                        } else if (a.res_mode == 3) {
-                            constexpr uint32_t I_LBO = ((uint32_t)(IROWS * 16) >> 4) << 16;
-                            const uint32_t b_lo = ((smem_u32(ident) + (uint32_t)((N - 16 - 16 * kc) * 16)) >> 4) | I_LBO;
-                            const uint32_t a_lo = a_base + (uint32_t)(((1 * TWP + 1) * 16) >> 4);
+                        for (int tap = 0; tap < 9; tap++) {
+                            const int dy = tap / 3, dx = tap - dy * 3;
+                            const uint32_t b_lo = b_base + (uint32_t)(tap * (2 * N * 16) >> 4);
+                            const uint32_t a_lo = a_base + (uint32_t)(((dy * TWP + dx) * 16) >> 4);
                             if (nplanes == 2) umma_issue_tap<MT, 2, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, 1u);
                             else umma_issue_tap<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, 1u);
                         }
@@ -502,7 +405,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                                 else umma_issue_tap<MT, 1, (A_PLANE >> 4), ROWSTEP16, N>(acc0, a_lo, b_lo, DESC_HI, idesc, 1u);
                             }
                     }
-                    if (a.dbg_flags & 64) umma_commit_elect(scratch_bar);  // timing experiment: what does one more commit per stage cost?
                     if (q == KS - 1) umma_commit_elect(&empty[s]);  // frees the stage once the MMAs above have read it
                     if (dbg && it - dskip < 12u && lane == 0) dbg[32 + it - dskip] = clock64();
                     if (++q == KS) { q = 0; if (++s == NST) { s = 0; ph ^= 1; } }
@@ -520,16 +422,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
         const int q = warp & 3;  // TMEM lane quarter this warp may access
         const int ehalf = (warp - 2) >> 2;  // the two warps of a quarter take alternate channel blocks
         const int p = q * 32 + lane;  // flattened position inside an accumulator
-        const int xr = p & (TWP - 1), yrow = WIDE ? 0 : (p >> 6);
+        const int xr = p & (TWP - 1), yrow = p >> 6;
         uint32_t tcount = 0;
         const size_t HW = (size_t)a.H * a.W;
         for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, tcount++) {
             const int buf = tcount & 1;
             const uint32_t aph = (tcount >> 1) & 1;
-            const int teff = a.rev ? ntiles - 1 - tile : tile;
-            const int bimg = teff / tiles_img, trem = teff - bimg * tiles_img;
+            const int bimg = tile / tiles_img, trem = tile - bimg * tiles_img;
             const int tx = trem % a.tiles_x, ty = trem / a.tiles_x;
-            const int x0 = tx * TVALID, y0 = ty * (RPA * MT);
+            const int x0 = tx * TVALID, y0 = ty * (2 * MT);
             const int x = x0 + xr;
             const __half* res_b = a.res + (size_t)bimg * a.res_bstride;
             __half* out_b = a.out + (size_t)bimg * a.out_bstride;
@@ -545,14 +446,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                 const float2 sm1v = make_float2(sm1, sm1);
                 // per-thread output address pieces: block (m, cb) -> obase + m * mstep + cb * cbstep
                 const bool s2d = a.out_s2d != 0;
-                const int yb = y0 + yrow;  // row of accumulator 0; accumulator m is RPA rows further down each
+                const int yb = y0 + yrow;  // row of accumulator 0; accumulator m is 2 rows further down each
                 const size_t cg_stride = !s2d ? HW : (HW >> 2);
                 const size_t pix0 = !s2d ? (size_t)yb * a.W + x : (size_t)(yb >> 1) * (a.W >> 1) + (x >> 1);
                 const size_t cg_base = !s2d ? 0 : (size_t)((yb & 1) * 2 + (x & 1)) * a.out_cgroups;
                 __half* const obase = out_b + (cg_base * cg_stride + pix0) * 8;
-                static_assert(!WIDE || RPA == 1, "");
-                // (space-to-depth output: rows alternate between the two row-parity sub-images, so it needs 2-row accumulators)
-                const size_t mstep = (!s2d ? (size_t)RPA * a.W : (size_t)(a.W >> 1)) * 8;
+                const size_t mstep = (!s2d ? (size_t)2 * a.W : (size_t)(a.W >> 1)) * 8;
                 const size_t cbstep = (size_t)(CBL / 8) * cg_stride * 8, gstep = cg_stride * 8;
                 auto ldblk = [&](int blk, uint32_t* r) {
                     const int m = blk / NCBL, cb = blk - m * NCBL;
@@ -567,14 +466,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                 auto stblk = [&](int blk, const uint32_t* r, auto split_tag) {
                     constexpr bool SPLIT = decltype(split_tag)::value;
                     const int m = blk / NCBL, cb = blk - m * NCBL;
-                    if (!(xvalid && yb + RPA * m < a.H)) return;
-                    __half* op = obase + m * mstep + cb * cbstep;
-                    if constexpr (WIDE) {
-                        if (s2d) {  // one-row accumulators: consecutive accumulators alternate between the two row-parity sub-images
-                            const int y = yb + m;
-                            op = out_b + (((size_t)((y & 1) * 2 + (x & 1)) * a.out_cgroups) * cg_stride + (size_t)(y >> 1) * (a.W >> 1) + (x >> 1)) * 8 + cb * cbstep;
-                        }
-                    }
+                    if (!(xvalid && yb + 2 * m < a.H)) return;
+                    __half* const op = obase + m * mstep + cb * cbstep;
 #pragma unroll
                     for (int g = 0; g < CBL / 8; g++) {
                         uint32_t hw_[4], lw_[4];
@@ -603,7 +496,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                 mbar_wait(&acc_full[buf], aph);
                 tc_fence_after();
                 if (dbg && warp == 2 && lane == 0 && tcount - (uint32_t)a.dbg_skip < 4u) dbg[44 + 2 * (tcount - a.dbg_skip)] = clock64();
-                if (ehalf < NBLKL && !(a.dbg_flags & 8)) {
+                if (ehalf < NBLKL) {
                     ldblk(ehalf, ra);
 #pragma unroll 1
                     for (int blk = ehalf; blk < NBLKL; blk += 4) {
@@ -625,7 +518,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                 const bool has_res = a.res_mode != 0;
                 auto prefetch = [&](int blk, uint4* dst) {
                     const int m = blk / NCB, cb = blk % NCB;
-                    const int y = y0 + RPA * m + yrow;
+                    const int y = y0 + 2 * m + yrow;
                     if (!has_res || !xvalid || y >= a.H) return;
 #pragma unroll
                     for (int g = 0; g < G; g++) {
@@ -636,7 +529,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_conv3x3_kernel(const __grid_co
                 };
                 auto process = [&](int blk, const uint4* rcur) {
                     const int m = blk / NCB, cb = blk % NCB;
-                    const int y = y0 + RPA * m + yrow;
+                    const int y = y0 + 2 * m + yrow;
                     const bool valid = xvalid && y < a.H;
                     const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16) + buf * ACC_COLS + m * N + cb * CB;
                     const size_t pix = !a.out_s2d ? (size_t)y * a.W + x : (size_t)(y >> 1) * (a.W >> 1) + (x >> 1);
@@ -834,38 +727,31 @@ static EncodeTiledFn get_encode() {
     return fn;
 }
 
-template <int N, int MT, int STAGES, int TAPS, int WIDE = 0>
+template <int N, int MT, int STAGES, int TAPS>
 static int launch_t(const TcConvArgs& a_in, const CUtensorMap& tm, cudaStream_t st) {
     TcConvArgs a = a_in;
-    constexpr int TWP = WIDE ? 128 : 64;
-    constexpr int ROWS = TAPS == 5 ? 2 * MT : (WIDE ? 1 : 2) * MT + 2;
+    constexpr int TWP = 64;
+    constexpr int ROWS = TAPS == 5 ? 2 * MT : 2 * MT + 2;
     constexpr int A_PLANE = 2 * ROWS * TWP * 16;
     constexpr int W_BYTES = TAPS * 2 * N * 16;
     const int nplanes = a.split_in ? 2 : 1;
     // barriers etc. (256) + slope_s + ones tile (4 KB) + bias B matrix + identity matrix (res_mode 3, or resident weights)
     const size_t consts = 1024 + 256 + N * sizeof(float) + 2 * 128 * 16 + (size_t)2 * N * 16;
+    // The identity tap uses 512 B of this; shrinking the reservation would change stages / ks of some layers (to be measured).
     const size_t ident_bytes = (size_t)2 * (2 * N - 16) * 16;
     // resident weights (stride-1 kernels): the whole packed layer next to activation-only stages, when it fits
-    static const bool wres_ok = !(getenv("RIFE_B200_WRES") && atoi(getenv("RIFE_B200_WRES")) == 0);
     const size_t w_all = (size_t)(a.Cin / 16) * W_BYTES * (TAPS == 5 ? 5 : 1);
     const size_t budget = 227 * 1024;
     const size_t stage_a = (size_t)((A_PLANE * nplanes + 1023) & ~1023), stage_aw = (size_t)((A_PLANE * nplanes + W_BYTES + 1023) & ~1023);
     // resident weights need at least STAGES activation-only stages next to the whole layer
-    a.wres = wres_ok && TAPS == 9 && ((STAGES * stage_a + consts + ident_bytes + 127) & ~(size_t)127) + w_all <= budget;
-    // chunks per pipeline stage (RIFE_B200_KS, default TC_KS_DEFAULT): resident-weight kernels only, KC divisible, >= 2 stages left
-    static const int ks_env = getenv("RIFE_B200_KS") ? atoi(getenv("RIFE_B200_KS")) : TC_KS_DEFAULT;
+    a.wres = TAPS == 9 && ((STAGES * stage_a + consts + ident_bytes + 127) & ~(size_t)127) + w_all <= budget;
+    // chunks per pipeline stage: resident-weight kernels only, KC divisible, >= 2 stages left
     const size_t fixed = a.wres ? consts + ident_bytes + 127 + w_all : consts + (a.res_mode == 3 ? ident_bytes : 0);
-    static const int chunk_env = getenv("RIFE_B200_CHUNK_ISSUE") ? atoi(getenv("RIFE_B200_CHUNK_ISSUE")) : TC_CHUNK_ISSUE_DEFAULT;
-    a.chunk_issue = chunk_env;
-    static const int krot_env = getenv("RIFE_B200_KROT") ? atoi(getenv("RIFE_B200_KROT")) : TC_KROT_DEFAULT;
-    a.krot = (!a.wres && krot_env) ? 1 : 0;
     a.ks = 1;
-    if (a.wres && ks_env > 1 && (a.Cin / 16) % ks_env == 0 && (budget - fixed) / (stage_a * ks_env) >= 2) a.ks = ks_env;
+    if (a.wres && (a.Cin / 16) % TC_KS_DEFAULT == 0 && (budget - fixed) / (stage_a * TC_KS_DEFAULT) >= 2) a.ks = TC_KS_DEFAULT;
     const int stage_bytes = (int)(a.wres ? stage_a * a.ks : stage_aw);
     // pipeline depth: what shared memory allows (the stages are what hides the L2 / HBM latency of the activation tiles)
-    static const int max_stages = getenv("RIFE_B200_STAGES") ? atoi(getenv("RIFE_B200_STAGES")) : 8;
     int nst = (int)((budget - fixed) / stage_bytes);
-    if (nst > max_stages) nst = max_stages;
     if (nst > 8) nst = 8;
     if (nst < STAGES && a.ks == 1) nst = STAGES;
     a.stages = nst;
@@ -880,13 +766,13 @@ static int launch_t(const TcConvArgs& a_in, const CUtensorMap& tm, cudaStream_t 
     {
         std::lock_guard<std::mutex> lk(configured_mu);
         if (smem > configured[dev]) {
-            if (cudaFuncSetAttribute(tc_conv3x3_kernel<N, MT, STAGES, TAPS, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -3;
+            if (cudaFuncSetAttribute(tc_conv3x3_kernel<N, MT, STAGES, TAPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return -3;
             configured[dev] = smem;
         }
     }
     int ntiles = a.tiles_x * a.tiles_y * a.batch;
     int grid = ntiles < a.num_sms ? ntiles : a.num_sms;
-    tc_conv3x3_kernel<N, MT, STAGES, TAPS, WIDE><<<grid, NTHREADS, smem, st>>>(tm, a);
+    tc_conv3x3_kernel<N, MT, STAGES, TAPS><<<grid, NTHREADS, smem, st>>>(tm, a);
     g_launch_count++;
     return 0;
 }
@@ -895,9 +781,6 @@ int tc_conv_tile_rows(int N) { return N <= 64 ? 8 : (N <= 128 ? 4 : 2); }  // 2 
 
 template <int N, int MT, int STAGES>
 static int launch_n(const TcConvArgs& a, const CUtensorMap& tm, cudaStream_t st) {
-    if constexpr (N == 64) {  // the instance tc_wide_enabled() admits
-        if (a.wide) return launch_t<N, MT, STAGES, 9, 1>(a, tm, st);
-    }
     if constexpr (N == 48 || N == 96 || N == 128 || N == 192) {  // the widths of the 5x5 residual blocks (rife / HD / UHD / anime flownets)
         if (a.k5) return launch_t<N, MT, 2, 5>(a, tm, st);
     }
@@ -911,11 +794,8 @@ int launch_tc_conv(TcConvArgs a, const void* in, cudaStream_t st) {
     if (a.Cin % 16 || a.N % 16 || a.N < 16 || a.N > 256) return -4;
     const int nplanes = a.split_in ? 2 : 1;
     const int MT = tc_conv_tile_rows(a.N) / 2;
-    // wide tiles (one-row accumulators of 128 pixels, MT rows x 126 columns): stride-1 convolutions whose weights were packed
-    // for them (tc_wide_enabled)
-    a.wide = (!a.s2 && !a.k5 && a.epi == TC_EPI_C8 && tc_wide_enabled(a.N)) ? 1 : 0;  // must equal the packers' choice (pack_conv3x3_weights)
     if (a.k5 && (a.s2 || a.epi != TC_EPI_C8)) return -4;
-    const int TWP = a.wide ? 128 : 64, TVALID = TWP - (a.k5 ? 4 : 2), tile_rows = a.wide ? MT : 2 * MT;
+    const int TWP = 64, TVALID = TWP - (a.k5 ? 4 : 2), tile_rows = 2 * MT;
     a.tiles_x = (a.W + TVALID - 1) / TVALID;
     a.tiles_y = (a.H + tile_rows - 1) / tile_rows;
     if (!a.num_sms) a.num_sms = 148;
@@ -928,22 +808,16 @@ int launch_tc_conv(TcConvArgs a, const void* in, cudaStream_t st) {
     if (a.out_cgroups <= 0) a.out_cgroups = a.Cout / 8;  // a launch that writes a channel slice of a wider tensor sets it to the tensor's groups
     if (a.res_mode == 3) return -9;  // internal value, selected below
     // residual == the conv's own input (the ResConv blocks): let the tensor core add it (identity tap, see the kernel)
-    static const bool ident_ok = !(getenv("RIFE_B200_RES_IDENT") && atoi(getenv("RIFE_B200_RES_IDENT")) == 0);
-    if (ident_ok && a.res_mode == 1 && a.epi == TC_EPI_C8 && !a.s2 && !a.k5 && a.res == (const __half*)in && a.Cin == a.N && a.Cout == a.N && a.N <= 128 && (!a.res_split) == (!a.split_in) &&
+    if (a.res_mode == 1 && a.epi == TC_EPI_C8 && !a.s2 && !a.k5 && a.res == (const __half*)in && a.Cin == a.N && a.Cout == a.N && a.N <= 128 && (!a.res_split) == (!a.split_in) &&
         (!a.split_in || a.res_plane == (size_t)a.Cin * a.H * a.W) && (a.batch == 1 || a.res_bstride == a.in_bstride))
         a.res_mode = 3;
-    a.pair = (!a.s2 && !a.wide && !a.k5 && tc_pair_enabled(a.N)) ? 1 : 0;  // the weights were packed accordingly (pack_*_weights)
-    if (tc_pair_mode() & 2) a.pair |= 2;  // narrow identity tap for the self-residual layers (independent of the weight layout)
     const size_t img_bytes = (size_t)nplanes * cgroups * a.H * a.W * 16;
     if (a.batch > 1 && a.in_bstride * 2 < img_bytes) return -8;
-    // one pixel's 8 channels = 16 bytes = 4 u32 elements (64-pixel boxes) or 2 u64 elements (128-pixel boxes: a box dimension
-    // holds at most 256 elements)
-    const int epp = a.wide ? 2 : 4;
-    cuuint64_t dims[4] = {(cuuint64_t)a.W * epp, (cuuint64_t)a.H, (cuuint64_t)nplanes * cgroups, (cuuint64_t)a.batch};
+    cuuint64_t dims[4] = {(cuuint64_t)a.W * 4, (cuuint64_t)a.H, (cuuint64_t)nplanes * cgroups, (cuuint64_t)a.batch};
     cuuint64_t strides[3] = {(cuuint64_t)a.W * 16, (cuuint64_t)a.H * a.W * 16, a.batch > 1 ? (cuuint64_t)a.in_bstride * 2 : (cuuint64_t)img_bytes};
-    cuuint32_t box[4] = {(cuuint32_t)(TWP * epp), (cuuint32_t)(a.k5 ? tile_rows : tile_rows + 2), 2, 1};
+    cuuint32_t box[4] = {(cuuint32_t)(TWP * 4), (cuuint32_t)(a.k5 ? tile_rows : tile_rows + 2), 2, 1};
     cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&tm, a.wide ? CU_TENSOR_MAP_DATA_TYPE_UINT64 : CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, const_cast<void*>(in), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, const_cast<void*>(in), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return -5;
     switch (a.N) {
@@ -1018,37 +892,9 @@ void launch_c8_to_planar(const __half* in, float* out, int C, int H, int W, int 
 }
 
 // ---- weight packing (host) -----------------------------------------------------------------------
-// Paired MMA issue (kernel: a.pair), for every stride-1 layer whose 2N fits one MMA.  RIFE_B200_PAIR (bit 0: paired
-// issue + [dy2|dy0|dy1] weight blocks, bit 1: narrow identity tap; default TC_PAIR_DEFAULT) is read once per process;
-// packing and launching consult the same function, so they cannot disagree.
+// Paired MMA issue (tc_paired), for every stride-1 layer whose 2N fits one MMA.
 // Measured (profiles/README.md, round-1 session 20): 16-channel mainloop stage of the 64->64 layer 2306 -> 1979 cycles,
 // the layer itself 96.5 -> 84.2 us at 8 x 480x272, whole model 2195 -> 2311 frames/s at 1080p.
-int tc_pair_mode() {
-    static const int mode = getenv("RIFE_B200_PAIR") ? atoi(getenv("RIFE_B200_PAIR")) & 3 : TC_PAIR_DEFAULT;
-    return mode;
-}
-bool tc_pair_enabled(int N) { return (tc_pair_mode() & 1) && 2 * N <= 256; }
-// Wide tiles (kernel template WIDE; RIFE_B200_WIDE, default TC_WIDE_DEFAULT): stride-1 convolutions with N = 64 -- the residual
-// chain of IFBlock 3, 44 % of the model's FLOPs.  (3N <= 256 would also admit N = 32 / 48; those layers run on maps too narrow
-// for 126-column tiles to pay.)  Packers and launcher consult the same function.
-bool tc_wide_enabled(int N) {
-    static const int on = getenv("RIFE_B200_WIDE") ? atoi(getenv("RIFE_B200_WIDE")) : TC_WIDE_DEFAULT;
-    return on && N == 64;
-}
-// [kc][tap = dy*3+dx][half][N][8] -> [kc][dx][half][3N rows: dy2 | dy1 | dy0][8]
-static void to_wide_layout(std::vector<uint16_t>& w, int kcs, int N) {
-    std::vector<uint16_t> o(w.size());
-    for (int kc = 0; kc < kcs; kc++)
-        for (int dy = 0; dy < 3; dy++)
-            for (int dx = 0; dx < 3; dx++)
-                for (int hf = 0; hf < 2; hf++)
-                    for (int n = 0; n < N; n++) {
-                        const size_t src = ((((size_t)kc * 9 + dy * 3 + dx) * 2 + hf) * N + n) * 8;
-                        const size_t dst = ((((size_t)kc * 3 + dx) * 2 + hf) * (3 * N) + (size_t)(2 - dy) * N + n) * 8;
-                        for (int j = 0; j < 8; j++) o[dst + j] = w[src + j];
-                    }
-    w.swap(o);
-}
 // [kc][tap = dy*3+dx][half][N][8] -> [kc][dx][half][3N rows: dy2 | dy0 | dy1][8]
 static void to_paired_layout(std::vector<uint16_t>& w, int kcs, int N) {
     std::vector<uint16_t> o(w.size());
@@ -1076,9 +922,7 @@ void pack_conv3x3_weights(const float* w, int cout, int cin, int N, std::vector<
                         __half h = __float2half_rn(w[((size_t)n * cin + ic) * 9 + tap]);
                         out[((((size_t)kc * 9 + tap) * 2 + hf) * N + n) * 8 + j] = __half_as_ushort(h);
                     }
-    // paired: -1 = what the launcher will assume for a stride-1 conv of this N; 0 plain; 1 paired; 2 wide
-    if (paired == 2 || (paired < 0 && tc_wide_enabled(N))) { if (3 * N <= 256) to_wide_layout(out, cin / 16, N); }
-    else if (paired < 0 ? tc_pair_enabled(N) : (paired != 0 && 2 * N <= 256)) to_paired_layout(out, cin / 16, N);
+    if (paired != 0 && tc_paired(N)) to_paired_layout(out, cin / 16, N);  // -1: what the launcher assumes; 1: paired where it fits
 }
 // conv 5x5 stride 1: w[oc][ic][5][5] fp32 (fp16-exact) -> wpk[kc][dy][dx][half][n][8]: one kernel row (five taps) per pipeline stage
 void pack_conv5x5_weights(const float* w, int cout, int cin, int N, std::vector<uint16_t>& out) {
@@ -1134,7 +978,7 @@ void pack_deconv4x4_weights(const float* w, int cout, int cin, int ocs, int N, s
                                 out[((((size_t)kc * 9 + dy * 3 + dx) * 2 + hf) * N + par * ocs + oc) * 8 + j] = __half_as_ushort(h);
                             }
                 }
-    if (paired < 0 ? tc_pair_enabled(N) : (paired != 0 && 2 * N <= 256)) to_paired_layout(out, cin / 16, N);
+    if (paired != 0 && tc_paired(N)) to_paired_layout(out, cin / 16, N);
 }
 
 }  // namespace rife

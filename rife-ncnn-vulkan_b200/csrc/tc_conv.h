@@ -35,36 +35,24 @@ struct TcConvArgs {
     int out_cgroups;        // 8-channel groups of the output TENSOR (0 = Cout / 8); larger when this launch writes a channel slice of it
     int tiles_x, tiles_y, num_sms;  // filled by the launcher
     int stages;                     // filled by the launcher: pipeline depth (<= 8)
-    int chunk_issue;                // filled by the launcher: all MMAs of a 16-channel chunk from one asm block (RIFE_B200_CHUNK_ISSUE)
-    int rev;                        // walk the tiles in reverse raster order (alternated by the caller across the layers of a chain: L2 reuse)
-    int krot;                       // filled by the launcher: per-CTA rotation of the K loop (streamed-weight kernels; RIFE_B200_KROT)
-    int ks;                         // filled by the launcher: 16-channel chunks per pipeline stage (resident-weight kernels; RIFE_B200_KS)
+    int ks;                         // filled by the launcher: 16-channel chunks per pipeline stage (resident-weight kernels)
     int wres;                       // filled by the launcher: the layer's packed weights stay resident in shared memory
-    int wide;                       // filled by the launcher: one-row accumulators / 126-column tiles (tc_wide_enabled)
-    int pair;                       // filled by the launcher: bit 0 paired MMA issue over [dy2 | dy0 | dy1] weight blocks (tc_pair_enabled), bit 1 narrow identity tap
     unsigned long long* dbg;        // optional timeline buffer: 64 clock64 slots per CTA (diagnostics)
     int dbg_skip;                   // tiles (per CTA) to skip before the timeline starts recording
-    int dbg_flags;                  // timing experiments only (results wrong): 1 = no identity tap, 2 = no bias MMAs after the first tiles, 4 = a third of the taps, 8 = empty epilogue, 16 = no activation / weight loads, 64 = one extra tcgen05.commit per stage
 };
 
 // `in`: C8 planar activation [planes][Cin/8][H][W][8] fp16.  Returns 0 on success.
 int launch_tc_conv(TcConvArgs a, const void* in, cudaStream_t st);
 int tc_conv_tile_rows(int N);
-// Paired MMA issue for stride-1 layers with 2N <= 256 (environment RIFE_B200_PAIR: bit 0 paired issue, bit 1 narrow
-// identity tap; default TC_PAIR_DEFAULT): the weight packers and the launcher both consult it.
-constexpr int TC_PAIR_DEFAULT = 3;
-int tc_pair_mode();
-bool tc_pair_enabled(int N);
-constexpr int TC_CHUNK_ISSUE_DEFAULT = 1;
-constexpr int TC_KROT_DEFAULT = 0;
+// Paired MMA issue over [dy2 | dy0 | dy1] weight blocks for every stride-1 layer whose 2N columns fit one MMA: the weight
+// packers and the launcher both decide the layout here.
+__host__ __device__ constexpr bool tc_paired(int N) { return 2 * N <= 256; }
 constexpr int TC_KS_DEFAULT = 2;  // measured (profiles/r2_s6): chain of IFBlock 3 704 -> 692 us, IFBlock 2 414 -> 403 us per 8 launches
-constexpr int TC_WIDE_DEFAULT = 0;  // measured slower than the paired 2-row form (profiles/README.md, round 2 session 2): 739 vs 687 us per 8 launches
-bool tc_wide_enabled(int N);
 
 void launch_planar_to_c8(const float* in, __half* out, int C, int H, int W, int split, cudaStream_t st, int Cpad = 0, int s2d = 0);
 void launch_c8_to_planar(const __half* in, float* out, int C, int H, int W, int split, cudaStream_t st, int Cpad = 0, int s2d = 0);
 
-// paired: -1 = what the launcher will assume for this N (tc_wide_enabled / tc_pair_enabled), 0 plain / 1 paired / 2 wide = explicit (diagnostics)
+// paired: -1 = what the launcher will assume for this N (tc_paired), 0 plain / 1 paired (if 2N <= 256) = explicit (diagnostics)
 void pack_conv3x3_weights(const float* w, int cout, int cin, int N, std::vector<uint16_t>& out, int paired = -1);
 void pack_conv5x5_weights(const float* w, int cout, int cin, int N, std::vector<uint16_t>& out);
 void pack_conv3x3s2_weights(const float* w, int cout, int cin, int cinp, int N, std::vector<uint16_t>& out);

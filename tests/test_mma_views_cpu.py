@@ -2,10 +2,14 @@
 descriptors (row i of an operand = 16 contiguous bytes at start + i*16, second K half LBO bytes further) applied to
 (a) the real packed weights (rife_b200_debug_pack_weights) and (b) a halo tile laid out as TMA delivers it, with the
 exact start-address / TMEM-column arithmetic of the kernel's issue loops.  The unpaired issue order is the one verified
-on the GPU (tests/test_tc_conv_gpu.py); the paired order (RIFE_B200_PAIR: one 2N-column MMA feeds the dy=2 tap of
-accumulator j-1 and the dy=0 tap of accumulator j) must produce the same accumulators, and both must equal a direct
-3x3 convolution / 4x4 stride-2 deconvolution of the tile."""
+on the GPU (tests/test_tc_conv_gpu.py); the paired order of umma_issue_chunk_paired (tools/gen_mma_issue.py chunk_block:
+per kernel column dx the paired rows -- one 2N-column MMA feeds the dy=2 tap of accumulator j-1 and the dy=0 tap of
+accumulator j -- then the dy=1 taps; the identity tap comes last and is not replayed here) must produce the same
+accumulators, and both must equal a direct 3x3 convolution / 4x4 stride-2 deconvolution of the tile.
+The generated issue code itself must be what tools/gen_mma_issue.py produces."""
 import ctypes
+import importlib.util
+import os
 
 import numpy as np
 import pytest
@@ -56,7 +60,7 @@ def _accumulate(slabs, wpk, N, MT, paired):
         else:
             for dx in range(3):
                 blk = dx * 2 * 3 * N  # 16-byte rows from the chunk start
-                for j in range(MT + 1):  # even views (umma_issue_pair)
+                for j in range(MT + 1):  # even views: paired rows
                     A = _a_view(slab, rows, dx + j * rowstep)
                     if j == 0:
                         acc[:, 0:N] += A @ _b_view(wk[kc], blk + N, 3 * N, N).T
@@ -64,7 +68,7 @@ def _accumulate(slabs, wpk, N, MT, paired):
                         acc[:, (MT - 1) * N:MT * N] += A @ _b_view(wk[kc], blk, 3 * N, N).T
                     else:
                         acc[:, (j - 1) * N:(j + 1) * N] += A @ _b_view(wk[kc], blk, 3 * N, 2 * N).T
-                for m in range(MT):  # odd views (umma_issue_tap at one row down, dy = 1 rows of the block)
+                for m in range(MT):  # odd views (one row down, dy = 1 rows of the block)
                     A = _a_view(slab, rows, dx + TWP + m * rowstep)
                     acc[:, m * N:(m + 1) * N] += A @ _b_view(wk[kc], blk + 2 * N, 3 * N, N).T
     return acc.reshape(128, MT, N).transpose(1, 0, 2)
@@ -122,47 +126,21 @@ def test_deconv_views_paired_equals_unpaired(pkg):
             assert abs(a1[m, p, par * ocs + oc] - s) < 1e-3, (par, oc, a1[m, p, par * ocs + oc], s)
 
 
-# ---- wide tiles (kernel template WIDE): one-row accumulators of 128 pixels, [dy2 | dy1 | dy0] weight blocks ------------------
-WTW = 128
+def test_pack_weights_rejects_unknown_layout(pkg):
+    """paired is -1 (the kernel's layout for this N), 0 or 1; anything else is an argument error."""
+    w = np.zeros((16, 16, 3, 3), np.float32)
+    out = np.zeros(9 * 2 * 16 * 8, np.uint16)
+    for paired in (-2, 2, 3):
+        assert pkg.lib().rife_b200_debug_pack_weights(0, 16, 16, 16, 0, paired, w.ctypes.data, out.ctypes.data, out.size) != 0, paired
+    assert pkg.lib().rife_b200_debug_pack_weights(0, 16, 16, 16, 0, -1, w.ctypes.data, out.ctypes.data, out.size) == 0
 
 
-def _a_view_wide(slab, rows, start16):
-    """A operand (128 x 16) from a wide slab [2 halves][rows][128 px][8]: 128 consecutive pixels from start16 (wraps into the
-    next row for dx > 0; behind the last row: the overrun pad)."""
-    flat = slab.reshape(2, rows * WTW, 8)
-    flat = np.concatenate([flat, np.zeros((2, 64, 8), np.float32)], axis=1)
-    return np.concatenate([flat[0, start16:start16 + 128], flat[1, start16:start16 + 128]], axis=1)
-
-
-def _accumulate_wide(slabs, wpk, N, MT):
-    """umma_issue_wide (tools/gen_mma_issue.py wide_block): per kernel column dx, halo row r feeds accumulators r - dy."""
-    rows = MT + 2
-    kcs = len(slabs)
-    acc = np.zeros((128, MT * N), np.float64)
-    wk = wpk.reshape(kcs, -1)
-    for kc in range(kcs):
-        for dx in range(3):
-            blk = dx * 2 * 3 * N
-            for r in range(MT + 2):
-                dy_max, dy_min = min(2, r), max(0, r - (MT - 1))
-                ncol = (dy_max - dy_min + 1) * N
-                A = _a_view_wide(slabs[kc], rows, dx + r * WTW)
-                B = _b_view(wk[kc], blk + (2 - dy_max) * N, 3 * N, ncol)
-                c0 = (r - dy_max) * N
-                acc[:, c0:c0 + ncol] += A @ B.T
-    return acc.reshape(128, MT, N).transpose(1, 0, 2)
-
-
-@pytest.mark.parametrize("cin,cout,N,MT", [(64, 64, 64, 4), (32, 64, 64, 4)])
-def test_conv3x3_wide_views_equal_direct(pkg, cin, cout, N, MT):
-    rng = np.random.default_rng(cin + 3 * N)
-    w = (rng.standard_normal((cout, cin, 3, 3)) * 0.1).astype(np.float16).astype(np.float32)
-    rows = MT + 2
-    x = rng.standard_normal((cin, rows, WTW)).astype(np.float16).astype(np.float32)
-    slabs = [x[kc * 16:(kc + 1) * 16].reshape(2, 8, rows, WTW).transpose(0, 2, 3, 1).copy() for kc in range(cin // 16)]
-    acc = _accumulate_wide(slabs, _pack(pkg, 0, w, cout, cin, N, 0, 2), N, MT)
-    for m in range(MT):  # position p of accumulator m: output row m, column p (valid < 126)
-        for p in range(0, WTW - 2, 7):
-            patch = x[:, m:m + 3, p:p + 3]
-            want = np.tensordot(w, patch, axes=([1, 2, 3], [0, 1, 2]))
-            assert np.allclose(acc[m, p, :cout], want, atol=1e-3), (m, p)
+def test_generated_mma_issue_is_current(tmp_path):
+    """csrc/tc_mma_issue.inc is the output of tools/gen_mma_issue.py (an edit of either alone does not pass)."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("gen_mma_issue", os.path.join(root, "tools", "gen_mma_issue.py"))
+    gen = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(gen)
+    out = tmp_path / "tc_mma_issue.inc"
+    gen.main(str(out))
+    assert out.read_text() == open(os.path.join(root, "rife-ncnn-vulkan_b200", "csrc", "tc_mma_issue.inc")).read()

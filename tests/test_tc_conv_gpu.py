@@ -96,10 +96,9 @@ def test_conv3x3_stride2(pkg, cin, cout):
 @pytest.mark.parametrize("split", [1, 0])
 @pytest.mark.parametrize("self_res", [True, False])
 @pytest.mark.parametrize("h,w", [(11, 140), (4, 126), (5, 127), (9, 300)])
-def test_conv3x3_wide_tiles(pkg, h, w, self_res, split):
-    """N = 64 runs on the wide-tile variant (one-row accumulators of 128 pixels, 126 valid columns, rows in groups of 4; one
-    MMA of up to 192 columns feeds three accumulators): several column tiles, ragged last column and row tiles, the
-    self-residual identity tap and the epilogue residual."""
+def test_conv3x3_n64_ragged_tiles(pkg, h, w, self_res, split):
+    """N = 64 on the paired whole-chunk issue path (tiles of 8 rows x 62 columns): several column tiles, ragged last column
+    and row tiles, the self-residual identity tap and the epilogue residual."""
     c = 64
     x, wgt, b, res = _data(c, c, h, w, 9, seed=h * 1000 + w)
     x = np.ascontiguousarray(x, np.float32)
